@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W [--model v8n|v8s|v8x|...] [--batch B] [--gather comm|nccl]
     torchrun --nproc-per-node N bench.py --gpus N ...           (one rank per GPU)
     python bench.py --impl reference ...                         (the reference's CPU path, see below)
+    python bench.py ... --dump-outputs DIR                       (also write the last timed step's outputs as DIR/*.npy)
 
 One "step" = one pass of the hot path over one batch per GPU: yb_forward (tcgen05 fp16 network + DFL/box
 decode) -> yb_nms (GPU NMS) [-> all-gather of the fixed-capacity detection payloads when N > 1: by default the
@@ -46,6 +47,24 @@ E2E_SLOTS = 3  # batches in flight through yb_predict_u8_submit/_wait
 MASK_CAP = 32  # segment e2e: instance masks returned per image (byte planes of 640x640)
 # compulsory bytes per image, fp16 input + fp32 prediction tensor (SURVEY.md section 8(d))
 COMPULSORY_MB_IMG = {"detect": 3.87, "segment": 6.0}
+# --dump-outputs: an output with more elements is written as a sample of this many; keeps a dump well under 64 MB
+DUMP_SAMPLE = 1 << 20
+
+
+def dump_outputs(out_dir, outputs):
+    """Write each output of the last timed step as <out_dir>/<name>.npy, float32 (float64 for integer outputs).  An output
+    of more than DUMP_SAMPLE elements becomes <name>_sample.npy: its values at DUMP_SAMPLE flat positions drawn with a
+    fixed seed, in increasing order, so that two runs with the same arguments write files that compare element for element."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+            t, name = t.reshape(-1)[idx.to(t.device)], name + "_sample"
+        t = t.to(torch.float32 if t.is_floating_point() else torch.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 def load_peaks():
@@ -242,7 +261,7 @@ def train_main(args, rank, world, local_rank):
             opt.step()
         for _ in range(min(args.warmup, 1)):
             step()
-        n = max(1, min(args.steps, 3))
+        n = args.steps
         t0 = time.perf_counter()
         for _ in range(n):
             step()
@@ -295,6 +314,8 @@ def train_main(args, rank, world, local_rank):
             print(f"step {i}: {(time.perf_counter() - _t0) * 1e3:.1f} ms", file=sys.stderr)
     e1.record()
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:  # the step hands its caller the loss items and leaves the updated weights
+        dump_outputs(args.dump_outputs, {"loss_items": items, "weights": st.flat if native else st.P.flat})
     if world > 1:
         dist.barrier()
     t = torch.tensor([e0.elapsed_time(e1)], device=dev)
@@ -383,7 +404,14 @@ def main():
                     help="train: one YOLOv11s training step (fwd + v8DetectionLoss + bwd + all-reduce + AdamW), BASELINE configs[3]")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-real-weights", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (inputs are seeded, so two "
+                         "builds run with the same arguments can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -442,10 +470,11 @@ def main():
     A, Cp = eng.anchors, eng.pred_channels
     gatherer = ydist.DetectionGather(B, MAX_DET, ROW, dev, mode=args.gather, slots=max(2, E2E_SLOTS)) if world > 1 else None
 
-    def timed_run(eng, xs, steps, warmup, with_gather):
+    def timed_run(eng, xs, steps, warmup, with_gather, snapshot=False):
         """Two-deep software pipeline: forward(i+1) runs on stream s_f while NMS (+ masks, + gather) of batch i runs on
         stream s_n, each with its own prediction / detection buffers - every step does all of its work inside the
-        timed region.  Returns (ms_total over `steps`, mean detections per image, last pred buffer)."""
+        timed region.  Returns (ms_total over `steps`, mean detections per image, last pred buffer, forward-only ms per
+        step, the last timed step's outputs if `snapshot` else None)."""
         s_f, s_n = torch.cuda.Stream(dev, priority=-1), torch.cuda.Stream(dev, priority=-1)
         preds = [torch.empty((B, Cp, A), dtype=torch.float32, device=dev) for _ in range(2)]
         protos = [torch.empty((B, 32, 160, 160), dtype=torch.float32, device=dev) for _ in range(2)] if seg else None
@@ -484,6 +513,16 @@ def main():
         s_f.wait_stream(s_n)
         e1.record(s_f)
         torch.cuda.synchronize()
+        last = None
+        if snapshot:  # rows past an image's detection count hold stale data: they are not part of the result
+            b = (steps - 1) & 1
+            dets, counts = gatherer.gathered(b) if with_gather else detb[b][:2]  # all ranks' images when gathered
+            rows = torch.arange(MAX_DET, device=dev)
+            valid, local = rows < counts[:, None], rows < detb[b][1][:, None]
+            last = {"pred": preds[b].clone(), "detections": torch.where(valid[..., None], dets, 0.0), "counts": counts.clone(),
+                    "keep": torch.where(local, keepb[b], -1)}
+            if seg:
+                last["masks"] = mask_buf[b].masked_fill_(~local[:, :, None, None], 0)
         if world > 1:
             dist.barrier()
         t = torch.tensor([e0.elapsed_time(e1)], device=dev)
@@ -496,14 +535,18 @@ def main():
             eng.forward(xs[i % len(xs)], preds[i & 1], protos[i & 1] if seg else None, stream=s_f)
         f1.record(s_f)
         torch.cuda.synchronize()
-        return float(t.item()), float(detb[0][1].float().mean().item()), preds[0], f0.elapsed_time(f1) / steps
+        return float(t.item()), float(detb[0][1].float().mean().item()), preds[0], f0.elapsed_time(f1) / steps, last
 
     xs = [synth_image(B, 640, 640, seed=100 + rank * 8 + i, dtype=torch.float16).to(dev) for i in range(4)]
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
-    ms_total, mean_dets, pred, fwd_ms = timed_run(eng, xs, args.steps, args.warmup, world > 1)
+    ms_total, mean_dets, pred, fwd_ms, last = timed_run(eng, xs, args.steps, args.warmup, world > 1,
+                                                        snapshot=bool(args.dump_outputs) and rank == 0)
     clocks = sampler.stop() if sampler else None
+    if last is not None:
+        dump_outputs(args.dump_outputs, last)
+        del last
     value = world * B * args.steps / (ms_total / 1e3)
 
     # ---- the same measurement on the reference's shipped checkpoint + its test images (v8n detect only) ----
@@ -516,7 +559,7 @@ def main():
             eng_r = make_engine({k: torch.from_numpy(z[k]) for k in z.files})
             u8 = image_batch(B)
             xr = [torch.roll(u8, shifts=i, dims=0).to(dev) for i in range(4)]  # uint8 input: /255 fused into the stem
-            ms_r, dets_r, _, fwd_r = timed_run(eng_r, xr, max(10, args.steps // 2), args.warmup, False)
+            ms_r, dets_r, _, fwd_r, _ = timed_run(eng_r, xr, max(10, args.steps // 2), args.warmup, False)
             real = {"value": round(B * max(10, args.steps // 2) / (ms_r / 1e3), 1), "unit": "images/s",
                     "weights": "reference Yolov8n.bin (tests/golden/yolov8n_f16.npz)",
                     "inputs": "32 x 640x640 uint8 built from the reference's 5 test images (pad 114, rolled copies)",

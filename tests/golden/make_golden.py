@@ -9,7 +9,12 @@ binary:  python tests/golden/make_golden.py
   v8n_bus.npz       oracle outputs for that image: post-NMS rows, kept anchors, a strided sample of
                     the (1,84,6300) prediction tensor
   nms_cases.npz     synthetic NMS inputs + oracle outputs (ties, empty image, >max_det, class offsets)
+  shipped_bins.json size and SHA-256 of the shipped Yolov8n.bin, yolov11n.bin and yolov8n-seg.bin; their tensors,
+                    in file order, are the *_f16.npz fixtures, so tests rebuild each file from its npz and check it
+                    against these (tests/util.py shipped_bin)
 """
+import hashlib
+import json
 import os
 import sys
 
@@ -22,6 +27,8 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 from oracle import binfmt, ops, yolo  # noqa: E402
 
 REF = "/root/reference/YoloSharpDemo/Assets/"
+SHIPPED_BINS = (("Yolov8n.bin", "yolov8n_f16.npz"), ("yolov11n.bin", "yolov11n_f16.npz"),
+                ("yolov8n-seg.bin", "yolov8n-seg_f16.npz"))
 
 
 def nms_case(seed, B, nc, A, extra=0, score_scale=1.0, quant=None, frac=1.0):
@@ -79,6 +86,17 @@ def main():
                                           int(sp.get("frac", 1.0) * 1000)])
     np.savez_compressed(os.path.join(HERE, "nms_cases.npz"), **cases)
     print({k: v.tolist() for k, v in cases.items() if k.endswith("_counts")})
+    write_shipped_digests()
+
+
+def write_shipped_digests():
+    digests = {}
+    for f, npz in SHIPPED_BINS:
+        raw = open(REF + "PreTrainedModels/" + f, "rb").read()
+        digests[f] = {"npz": npz, "bytes": len(raw), "sha256": hashlib.sha256(raw).hexdigest()}
+    with open(os.path.join(HERE, "shipped_bins.json"), "w") as fh:
+        json.dump(digests, fh, indent=1)
+        fh.write("\n")
 
 
 if __name__ == "__main__":

@@ -10,7 +10,7 @@ import tempfile
 
 import pytest
 
-from tests.util import ROOT
+from tests.util import ROOT, shipped_bin
 
 
 def header_functions():
@@ -94,13 +94,11 @@ def test_bin_roundtrip(tmp_path):
     p = str(tmp_path / "w.bin")
     binfmt.write_bin(p, t)
     assert binfmt.read_bin(p) == t
-    golden = os.path.join(ROOT, "tests", "golden")
-    ref = "/root/reference/YoloSharpDemo/Assets/PreTrainedModels/Yolov8n.bin"
-    if os.path.exists(ref):
-        r = binfmt.read_bin(ref)
-        assert len(r) == 357
-        binfmt.write_bin(p, r)
-        assert open(p, "rb").read() == open(ref, "rb").read()
+    ref = shipped_bin(tmp_path, "Yolov8n.bin")
+    r = binfmt.read_bin(ref)
+    assert len(r) == 357
+    binfmt.write_bin(p, r)
+    assert open(p, "rb").read() == open(ref, "rb").read()
 
 
 @pytest.mark.parametrize("arch,task,size", [("v8", "detect", "n"), ("v8", "detect", "s"), ("v8", "detect", "m"),

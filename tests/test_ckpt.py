@@ -1,6 +1,6 @@
 """Native checkpoint reader / writer (csrc/ckpt.cu) against the independent Python reader (yolosharp_b200/binfmt.py),
-the committed copy of the reference's shipped Yolov8n.bin (tests/golden/yolov8n_f16.npz) and, when the reference tree is
-mounted, the shipped file itself (byte-exact round trip)."""
+the committed copy of the reference's shipped Yolov8n.bin (tests/golden/yolov8n_f16.npz) and the shipped file itself, rebuilt
+from that copy and checked against its SHA-256 (byte-exact round trip)."""
 import json
 import os
 import struct
@@ -9,12 +9,11 @@ import numpy as np
 import pytest
 import torch
 
-from tests.util import GOLDEN
+from tests.util import GOLDEN, shipped_bin
 from yolosharp_b200 import binfmt
 from yolosharp_b200 import engine as E
 from yolosharp_b200._lib import YbError
 
-REF_BIN = "/root/reference/YoloSharpDemo/Assets/PreTrainedModels/Yolov8n.bin"
 CODE = {torch.float16: 5, torch.float32: 6, torch.int64: 4, torch.int32: 3}
 
 
@@ -39,10 +38,10 @@ def test_bin_native_writer_equals_python_writer_and_reference_file(tmp_path):
     binfmt.write_bin(a, [(k, CODE[v.dtype], list(v.shape), v.numpy().tobytes()) for k, v in sd.items()])
     E.write_checkpoint_bin(b, sd)
     assert open(a, "rb").read() == open(b, "rb").read()
-    if os.path.exists(REF_BIN):  # authoring container only: the shipped file round-trips byte for byte
-        c = str(tmp_path / "c.bin")
-        E.write_checkpoint_bin(c, E.read_checkpoint(REF_BIN))
-        assert open(c, "rb").read() == open(REF_BIN, "rb").read()
+    ref = shipped_bin(tmp_path, "Yolov8n.bin")  # the shipped file round-trips byte for byte
+    c = str(tmp_path / "c.bin")
+    E.write_checkpoint_bin(c, E.read_checkpoint(ref))
+    assert open(c, "rb").read() == open(ref, "rb").read()
 
 
 def test_safetensors_reader(tmp_path):

@@ -1,5 +1,6 @@
-"""CPU tests: the oracle against its golden vectors, the reference's shipped assets (when the
-reference tree is mounted), and an independent NMS restatement.  No GPU, no product code."""
+"""CPU tests: the oracle against its golden vectors, the reference's shipped checkpoints (rebuilt from their golden
+copies and checked against the shipped files' SHA-256), and an independent NMS restatement.  No GPU, and no product
+code except the pure-Python .bin writer that rebuilds those checkpoints."""
 import os
 
 import numpy as np
@@ -7,10 +8,7 @@ import pytest
 import torch
 
 from oracle import binfmt, ops, yolo
-from tests.util import GOLDEN, golden_nms_cases, oracle_real_v8n
-
-REF = "/root/reference/YoloSharpDemo/Assets/"
-has_ref = os.path.isdir(REF)
+from tests.util import GOLDEN, golden_nms_cases, oracle_real_v8n, shipped_bin
 
 
 def test_nms_golden_and_independent_restatement():
@@ -72,20 +70,19 @@ def test_model_sizes_match_survey():
     assert abs(nparams(yolo.build("v11", "detect", "s")) / 1e6 - 9.459) < 0.01
 
 
-@pytest.mark.skipif(not has_ref, reason="reference tree not mounted (GPU box)")
-def test_bin_reader_on_shipped_checkpoints():
+def test_bin_reader_on_shipped_checkpoints(tmp_path):
     for arch, task, f, cnt in (("v8", "detect", "Yolov8n.bin", 357), ("v11", "detect", "yolov11n.bin", 501),
                                ("v8", "segment", "yolov8n-seg.bin", 419)):
-        sd, trailing = binfmt.load_bin(REF + "PreTrainedModels/" + f)
+        path = shipped_bin(tmp_path, f)
+        sd, trailing = binfmt.load_bin(path)
         assert trailing == 0 and len(sd) == cnt
         m = yolo.build(arch, task, "n")
-        missing, unexpected = binfmt.load_into(m, REF + "PreTrainedModels/" + f)
+        missing, unexpected = binfmt.load_into(m, path)
         assert missing == [] and unexpected == []
 
 
-@pytest.mark.skipif(not has_ref, reason="reference tree not mounted (GPU box)")
-def test_golden_weights_equal_shipped_checkpoint():
-    sd, _ = binfmt.load_bin(REF + "PreTrainedModels/Yolov8n.bin")
+def test_golden_weights_equal_shipped_checkpoint(tmp_path):
+    sd, _ = binfmt.load_bin(shipped_bin(tmp_path, "Yolov8n.bin"))
     z = np.load(os.path.join(GOLDEN, "yolov8n_f16.npz"))
     assert sorted(z.files) == sorted(sd.keys())
     for k in z.files:

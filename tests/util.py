@@ -1,4 +1,6 @@
 """Shared helpers for the parity tests (the oracle is the checker, never the thing measured)."""
+import hashlib
+import json
 import os
 import sys
 
@@ -69,6 +71,20 @@ def oracle_real_v8n():
     new = {k: torch.from_numpy(z[k].astype(np.float32)).reshape(own[k].shape) for k in z.files if k in own}
     m.load_state_dict(new, strict=False)
     return m, {k: torch.from_numpy(z[k]) for k in z.files}
+
+
+def shipped_bin(directory, name):
+    """The reference's shipped checkpoint `name` (Yolov8n.bin, yolov11n.bin or yolov8n-seg.bin), written into `directory`
+    from the golden copy of its tensors and checked byte for byte (size and SHA-256) against the shipped file.  -> path."""
+    from yolosharp_b200 import binfmt
+    spec = json.load(open(os.path.join(GOLDEN, "shipped_bins.json")))[name]
+    z = np.load(os.path.join(GOLDEN, spec["npz"]))
+    code = {np.dtype(np.float16): 5, np.dtype(np.float32): 6}
+    path = os.path.join(str(directory), name)
+    binfmt.write_bin(path, [(k, code[z[k].dtype], z[k].shape, z[k].tobytes()) for k in z.files])
+    raw = open(path, "rb").read()
+    assert len(raw) == spec["bytes"] and hashlib.sha256(raw).hexdigest() == spec["sha256"], f"{name} differs from the shipped file"
+    return path
 
 
 def oracle_activations(model, x):
